@@ -280,10 +280,12 @@ class DeviceLoop:
             self.last = (si, acc[j])
 
     def time_windows(self, steps, warmup, windows, pdl, graph, barrier=None, reduce_max=None):
-        """Returns per-window milliseconds (max over ranks when reduce_max is given) and the launches per window."""
+        """Returns per-window milliseconds (max over ranks when reduce_max is given) and the launches per window; the steps
+        evaluated inside the timed windows are counted in self.timed_steps."""
         torch, gf = self.torch, self.gf
         self.kern.set_launch_overlap(pdl)
         n_sets = len(self.d_pos)
+        self.timed_steps = 0
         with torch.cuda.stream(self.stream):
             done = 0
             while done < warmup:                      # untimed warm-up steps, in windows of at most K
@@ -311,6 +313,7 @@ class DeviceLoop:
                 if rendezvous:
                     self.comm.rendezvous(self.stream.cuda_stream, hold=True)
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                evals_before = sum(self.set_evals)
                 e0.record(self.stream)
                 if g is not None:
                     g.launch(self.stream.cuda_stream)
@@ -321,6 +324,7 @@ class DeviceLoop:
                 if rendezvous:
                     self.comm.rendezvous_release()
                 self.stream.synchronize()
+                self.timed_steps += sum(self.set_evals) - evals_before
                 if barrier is not None:
                     barrier()
                 out.append(e0.elapsed_time(e1))
@@ -429,7 +433,8 @@ def run_e2e(gf, kern, w, local_rank, steps, reduce_max_scalar=None, barrier=None
         secs = time_e2e(fn, steps, 3)
         if reduce_max_scalar is not None:
             secs = reduce_max_scalar(secs)
-        out[name] = {"ms_per_step": secs / steps * 1e3, "h2d_bytes_per_step": int(w.pos.nbytes), "d2h_bytes_per_step": int(d2h[name])}
+        out[name] = {"ms_per_step": secs / steps * 1e3, "timed_steps": steps, "h2d_bytes_per_step": int(w.pos.nbytes),
+                     "d2h_bytes_per_step": int(d2h[name])}
     # the energies the batched entry point returned last (energy-only call ran third, C ABI last): keep them for the check
     batch.evaluateWithForcesF32(pos_h, r, e_h, f32_h)
     result = (e_h.copy(), f32_h.copy())
@@ -437,7 +442,7 @@ def run_e2e(gf, kern, w, local_rank, steps, reduce_max_scalar=None, barrier=None
     return out, result
 
 
-def run_single_ligand(gf, dev, steps=2000):
+def run_single_ligand(gf, dev, steps):
     """configs[1]: one 47-atom ligand in three 208x278x231 grids, one evaluation per MD step through the host API
     (positions in, energy + forces out, synchronous). OpenMM's integrator is not available here, so the figure is the
     grid-force-limited upper bound: steps/s x 4 fs (example/input.json:24)."""
@@ -558,9 +563,8 @@ def run_other_workload(torch, gf, dev, stream, name, steps, warmup, windows, pea
         pos_h[...] = w.pos
         f_h, _t2 = pinned_array(w.pos.shape, np.float32)
         e_h, _t3 = pinned_array((w.n_replicas,))
-        e2e_steps = 10
-        secs = time_e2e(lambda: kern.execute_host(pos_h, forces=f_h, force_mode=gf.FORCE_F32_STORE, energies_out=e_h), e2e_steps, 3)
-        out["e2e"] = {"value": w.evals * e2e_steps / secs, "unit": UNIT, "h2d_bytes_per_step": int(w.pos.nbytes),
+        secs = time_e2e(lambda: kern.execute_host(pos_h, forces=f_h, force_mode=gf.FORCE_F32_STORE, energies_out=e_h), steps, 3)
+        out["e2e"] = {"value": w.evals * steps / secs, "unit": UNIT, "h2d_bytes_per_step": int(w.pos.nbytes),
                       "d2h_bytes_per_step": int(w.pos.nbytes // 2 + 8 * w.n_replicas), "api": "gfb_kernel_execute_host, FP32 forces"}
     del loop
     kern.close()
@@ -597,7 +601,6 @@ def cpu_baseline(w, target_seconds=12.0, n_sample=2048, check=None):
     produced: per replica |E - E_ref| <= max(1e-6 |E_ref|, 6e-8 sum|s v|), forces 1e-5 relative (max-norm)."""
     from oracle import bindings
     from openmmgridforce_b200 import workloads as W
-    bindings.build()
     checked = []
     for label, pos, en, f in (check or []):
         port = bindings.PortOracle(w.counts, w.spacing, w.origin, w.grids, w.scaling, oob_k=w.oob_k)
@@ -642,7 +645,6 @@ def reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    bindings.build()
     threads = os.cpu_count() or 1
     cfg = workload_config(args.gpus, args.scaling)
     passes = max(1, cfg["replicas_total"] // REPLICAS_TOTAL)      # weak scaling at N > 1: the 65,536 poses N times per step
@@ -688,7 +690,9 @@ def reference_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="K: the steps of every timed window (the headline times --windows windows of K steps; the other "
+                         "variants, the other workloads and the per-call e2e loops time K steps or calls each)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--scaling", default=os.environ.get("GFB_BENCH_SCALING", "strong"), choices=["strong", "weak"],
@@ -701,9 +705,15 @@ def main():
                          "result is checked against another method outside the timed region.")
     ap.add_argument("--windows", type=int, default=5, help="timed K-step windows (median reported)")
     ap.add_argument("--no-extras", action="store_true", help="skip C2/C3/C4/C5 variants and the CPU baseline (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR (N=1 only): energies.npy [replicas] float64 and "
+                         "forces.npy [replicas, atoms, 3] float32, 37.5 MB in all; the inputs are seeded, so two builds run "
+                         "with the same arguments can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     args.windows = max(args.windows, 1)
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "b200"):
+        raise SystemExit("--dump-outputs needs --gpus 1 and --impl b200")
 
     if args.impl == "reference":
         reference_arm(args)
@@ -778,6 +788,7 @@ def main():
     variants, launches = run_variants(loop, args.steps, args.warmup, args.windows, barrier, reduce_max,
                                       which=[v for v in VARIANTS if v[0] == head_name])
     headline = variants[head_name]
+    timed_steps = loop.timed_steps
     gather_check = None
     if world > 1:
         comm.gather_status()
@@ -793,6 +804,8 @@ def main():
             raise SystemExit(f"rank {rank}: energy gather ({gather_mode}) does not match the reference all-gather")
         gather_check = f"{gather_mode} gather == " + ("ncclAllGather via gfb_comm_all_gather" if gather_mode != "nccl" else "torch all_gather_into_tensor") + " (bit-identical, outside the timed region)"
     dev_sample = loop.last_step_results(1024)
+    # taken now (the later windows overwrite the buffers), written to disk after the last measurement
+    dump = loop.last_step_results(loop.r)[1:] if args.dump_outputs else None
     # this rank's own per-step time (not the max over ranks, no gather) for the roofline of ITS kernel
     saved_mode, loop.gather_mode = loop.gather_mode, "none"
     own_ms, _ = loop.time_windows(args.steps, 0, 3, True, args.steps > 1)
@@ -809,26 +822,23 @@ def main():
         w_weak, sets_weak, _ = pose_sets(W, rank, world, False, 2)
         comm_w_total = REPLICAS_PER_GPU * world
         loop_w = DeviceLoop(torch, gf, dev, kern, sets_weak, N_ATOMS, stream, comm=None, gather_mode="none", lo=0, total=0)
-        steps_w = max(4, min(args.steps, 40))
-        vw, _ = run_variants(loop_w, steps_w, 4, 3, barrier, reduce_max, which=(VARIANTS[0],))
+        vw, _ = run_variants(loop_w, args.steps, 4, 3, barrier, reduce_max, which=(VARIANTS[0],))
         weak = {"scaling": "weak", "replicas_total": comm_w_total, "ms_per_step": vw["pdl+graph"]["ms_per_step"],
                 "value": comm_w_total * N_ATOMS * N_GRIDS / (vw["pdl+graph"]["ms_per_step"] * 1e-3), "unit": UNIT,
                 "note": "65,536 replicas per GPU, no energy gather in this window"}
         del loop_w
 
     # ---- end to end --------------------------------------------------------------------------------------------------
-    e2e_steps = max(3, min(args.steps, 20))
-    e2e, e2e_result = run_e2e(gf, kern, w, local_rank, e2e_steps, reduce_max_scalar, barrier)
+    e2e, e2e_result = run_e2e(gf, kern, w, local_rank, args.steps, reduce_max_scalar, barrier)
     if barrier is not None:
         barrier()
     host_copy_after = dev.bench_host_copy(64 << 20, 5)
 
     extras = {}
     if rank == 0 and world == 1 and not args.no_extras:
-        x_steps = max(20, min(args.steps, 200))
         for name in ("C3", "C4", "C5_double", "C5_energy_only", "C5_bspline", "C5_tricubic"):
-            extras[name] = run_other_workload(torch, gf, dev, stream, name, x_steps, args.warmup, 3, peak_gbs, l2_gbs)
-        extras["C2"] = run_single_ligand(gf, dev)
+            extras[name] = run_other_workload(torch, gf, dev, stream, name, args.steps, args.warmup, 3, peak_gbs, l2_gbs)
+        extras["C2"] = run_single_ligand(gf, dev, args.steps)
     clocks = sampler.stop()
 
     evals_step_rank = w.n_replicas * N_ATOMS * N_GRIDS
@@ -849,7 +859,7 @@ def main():
         line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": headline["ms_per_step"], "higher_is_better": True, "scaling": cfg["scaling"], "vs_baseline": None,
                 "dtype": "f32 interpolation, f64 index/energy, i64 fixed-point forces", "data": "synthetic", "config": cfg,
-                "run": {"windows": headline["windows"], "min_ms_per_step": headline["min_ms_per_step"],
+                "run": {"windows": headline["windows"], "timed_steps": timed_steps, "min_ms_per_step": headline["min_ms_per_step"],
                         "max_ms_per_step": headline["max_ms_per_step"],
                         "launch": ("CUDA graph of the K-step loop; launches carry programmatic-dependent-launch edges (a step's "
                                    "blocks fetch positions/records and issue their force atomics during the previous step's "
@@ -892,6 +902,10 @@ def main():
             checks = [("device loop, last timed step (FIXED_ADD, PDL + graph)",) + dev_sample,
                       ("GridForceBatch::evaluateWithForcesF32", w.pos[:1024], e2e_result[0][:1024], e2e_result[1][:1024].astype(np.float64))]
             line["cpu_baseline"] = cpu_baseline(w, check=checks)
+        if dump is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "energies.npy"), dump[0])
+            np.save(os.path.join(args.dump_outputs, "forces.npy"), dump[1].astype(np.float32))
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if world > 1:
