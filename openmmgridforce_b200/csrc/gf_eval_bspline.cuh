@@ -42,11 +42,13 @@ __device__ __forceinline__ void bspline_weights(double fx, double fy, double fz,
 }
 
 // One lane's stencil out of its 256-byte smem region: 16 granules of 16 bytes, granule 4*i + r = row r of x-plane i,
-// stored at position (4*i + r) ^ (lane & 7). Value FP64 from the FP32 points, gradient FP32.
+// stored at position (4*i + r) ^ (lane & 7). Value FP64 from the FP32 points, gradient FP32 over the points minus the
+// stencil's first point (see bspline_interpolate: the error then scales with |grad V|, not with |V|).
 __device__ __forceinline__ void bspline_from_smem(unsigned rbase, unsigned sw, const BsWeights& w, double& val, float& gx,
                                                   float& gy, float& gz) {
     val = 0.0;
     gx = gy = gz = 0.f;
+    float ref = 0.f;
 #pragma unroll
     for (int i = 0; i < 4; i++) {
         double pv = 0.0;
@@ -55,20 +57,22 @@ __device__ __forceinline__ void bspline_from_smem(unsigned rbase, unsigned sw, c
         for (int r = 0; r < 4; r++) {
             float v[4];
             lds128(rbase + (((4u * i + r) << 4) ^ sw), v);
+            if (i == 0 && r == 0) ref = v[0];
             double rz = 0.0;
             float rzs = 0.f, drz = 0.f;
 #pragma unroll
             for (int k = 0; k < 4; k++) {
+                const float d = v[k] - ref;
                 rz = fma(w.bz[k], (double) v[k], rz);
-                rzs = fmaf((float) w.bz[k], v[k], rzs);
-                drz = fmaf(w.dbz[k], v[k], drz);
+                rzs = fmaf((float) w.bz[k], d, rzs);
+                drz = fmaf(w.dbz[k], d, drz);
             }
             pv = fma(w.by[r], rz, pv);
             pdy = fmaf(w.dby[r], rzs, pdy);
             pdz = fmaf((float) w.by[r], drz, pdz);
         }
         val = fma(w.bx[i], pv, val);
-        gx = fmaf(w.dbx[i], (float) pv, gx);
+        gx = fmaf(w.dbx[i], (float) (pv - (double) ref), gx);
         gy = fmaf((float) w.bx[i], pdy, gy);
         gz = fmaf((float) w.bx[i], pdz, gz);
     }
@@ -116,7 +120,8 @@ __global__ void __launch_bounds__(kBsBlock, GFB_BS_MINBLOCKS) gf_eval_bspline_ke
     const unsigned t = blockIdx.x * kBsBlock + tid;
     const unsigned total = (unsigned) p.total;
     const bool active = t < total;
-    if (p.energies_clear && t < (unsigned) (p.n_replicas * p.n_slots)) p.energies_clear[t] = 0.0;
+    if (p.energies_clear)   // grid-stride: with energy slots the next accumulator can have more entries than the launch has threads
+        for (unsigned c = t; c < (unsigned) (p.n_replicas * p.n_slots); c += gridDim.x * blockDim.x) p.energies_clear[c] = 0.0;
 
     // ---- who am I (as gf_eval_lines_kernel) ----------------------------------------------------------------------
     unsigned rep = 0, ia = t;

@@ -67,7 +67,8 @@ __global__ void __launch_bounds__(kBsF64Block, 6) gf_eval_bspline_f64_kernel(con
     const unsigned t = blockIdx.x * kBsF64Block + tid;
     const unsigned total = (unsigned) p.total;
     const bool active = t < total;
-    if (p.energies_clear && t < (unsigned) (p.n_replicas * p.n_slots)) p.energies_clear[t] = 0.0;
+    if (p.energies_clear)   // grid-stride: with energy slots the next accumulator can have more entries than the launch has threads
+        for (unsigned c = t; c < (unsigned) (p.n_replicas * p.n_slots); c += gridDim.x * blockDim.x) p.energies_clear[c] = 0.0;
 
     // ---- who am I (as gf_eval_bspline_kernel) --------------------------------------------------------------------
     unsigned rep = 0, ia = t;

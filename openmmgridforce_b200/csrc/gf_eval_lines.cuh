@@ -467,7 +467,8 @@ __global__ void __launch_bounds__(lines_block(NG), lines_blocks_per_sm(NG, PERSI
         asm volatile("griddepcontrol.wait;" ::: "memory");
         if (defer) flush_parked((unsigned) kDefer);
     }
-    if (!defer && p.energies_clear && t < (unsigned) (p.n_replicas * p.n_slots)) p.energies_clear[t] = 0.0;
+    if (!defer && p.energies_clear)   // grid-stride, as below: the next accumulator can outnumber the launch's threads
+        for (unsigned c = t; c < (unsigned) (p.n_replicas * p.n_slots); c += gridDim.x * blockDim.x) p.energies_clear[c] = 0.0;
     if (p.atom_energies && active) p.atom_energies[a] = e_total;   // uniform branch (never with p.defer)
     // Force writes. In a launch that carries the fused energy gather they come AFTER the energies and the block's gather
     // ticket (the ticket's fence then waits for the energy atomics only); otherwise right here.

@@ -164,7 +164,8 @@ __global__ void __launch_bounds__(kLinesF64Block, 6) gf_eval_lines_f64_kernel(co
 
     // ---- writes start here (programmatic dependent launch: wait for the previous grid) ---------------------------------
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (p.energies_clear && t < (unsigned) (p.n_replicas * p.n_slots)) p.energies_clear[t] = 0.0;
+    if (p.energies_clear)   // grid-stride: with energy slots the next accumulator can have more entries than the launch has threads
+        for (unsigned c = t; c < (unsigned) (p.n_replicas * p.n_slots); c += gridDim.x * blockDim.x) p.energies_clear[c] = 0.0;
     if (p.atom_energies && active) p.atom_energies[a] = e_total;
     auto write_forces = [&]() {   // deferred behind the gather ticket in a gather launch (see gf_eval_lines_kernel)
         const bool stage_f = FMODE == GFB_FORCE_F64_STORE && p.forces != nullptr && plain && (t - lane) + 32u <= total &&

@@ -196,9 +196,17 @@ __device__ __forceinline__ void trilinear(const C v[8], C fx, C fy, C fz, C& val
     const C vm = ay * vmm + fy * vmp;
     const C vp = ay * vpm + fy * vpp;
     val = ax * vm + fx * vp;
-    dx = vp - vm;
-    dy = (vmp - vmm) * ax + (vpp - vpm) * fx;
-    dz = ((v[1] - v[0]) * ay + (v[3] - v[2]) * fy) * ax + ((v[5] - v[4]) * ay + (v[7] - v[6]) * fy) * fx;
+    if constexpr (sizeof(C) == 4) {
+        // MIXED: the stored corners are differenced first, as dz is. vp - vm subtracts two rounded lerps of size |V|, so
+        // its error grows with |V| (a field C + noise loses digits in proportion to C); a difference of two nearby FP32
+        // corners is exact or nearly so, which leaves an error proportional to |grad V| * spacing.
+        dx = ((v[4] - v[0]) * az + (v[5] - v[1]) * fz) * ay + ((v[6] - v[2]) * az + (v[7] - v[3]) * fz) * fy;
+        dy = ((v[2] - v[0]) * az + (v[3] - v[1]) * fz) * ax + ((v[6] - v[4]) * az + (v[7] - v[5]) * fz) * fx;
+    } else {   // DOUBLE: the reference's expressions (:1066-1068)
+        dx = vp - vm;
+        dy = (vmp - vmm) * ax + (vpp - vpm) * fx;
+    }
+    dz =((v[1] - v[0]) * ay + (v[3] - v[2]) * fy) * ax + ((v[5] - v[4]) * ay + (v[7] - v[6]) * fy) * fx;
 }
 
 // MIXED mode energy path: the interpolated VALUE is formed in FP64 from the FP32-stored corners and the FP64
@@ -305,7 +313,9 @@ __device__ __forceinline__ void accumulate_inside(const GridView& G, const S v[8
 // per stencil, half of the FMAs on zero weights) and single 64-byte bricks (16x; a brick still cost 89 bytes of DRAM).
 //
 // Arithmetic: S = double -> everything FP64. S = float -> gradient FP32, interpolated VALUE FP64 from the FP32-stored
-// points and FP64 weights (same reasoning as trilinear_value_f64).
+// points and FP64 weights (same reasoning as trilinear_value_f64). The FP32 gradient sums run over the points minus the
+// stencil's first point `ref`: each axis's derivative weights sum to 0, so the result is the same in exact arithmetic,
+// but the rounding error then scales with the spread of the stencil (|grad V| * spacing) instead of with |V|.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void bspline_basis(double t, double b[4], double d[4]) {   // :54-63
     const double u = 1.0 - t, t2 = t * t, t3 = t2 * t;
@@ -344,10 +354,12 @@ __device__ __forceinline__ void bspline_interpolate(const GridView& G, int ix, i
     const size_t plane2 = (size_t) G.nc[1] * G.nc[2] * 64;    // records two x-planes further on
     val = 0.0;
     gx = gy = gz = (S) 0;
+    S ref = (S) 0;                // MIXED: the stencil's first point, subtracted in the FP32 gradient sums
 #pragma unroll
     for (int i = 0; i < 4; i++) {
         S v[16];
         load_brick(rec + (i >> 1) * plane2 + (i & 1) * 16, v);   // planes ix, ix+1 | ix+2, ix+3
+        if (!F64 && i == 0) ref = v[0];
         double pv = 0.0;          // sum over (j,k) of by*bz*V in this x-plane
         S pdy = (S) 0, pdz = (S) 0;
 #pragma unroll
@@ -356,9 +368,10 @@ __device__ __forceinline__ void bspline_interpolate(const GridView& G, int ix, i
             S rzs = (S) 0, drz = (S) 0;
 #pragma unroll
             for (int k = 0; k < 4; k++) {
+                const S d = F64 ? v[4 * r + k] : v[4 * r + k] - ref;
                 rz = fma(bz[k], (double) v[4 * r + k], rz);
-                if (!F64) rzs = fma((S) bz[k], v[4 * r + k], rzs);
-                drz = fma((S) dbz[k], v[4 * r + k], drz);
+                if (!F64) rzs = fma((S) bz[k], d, rzs);
+                drz = fma((S) dbz[k], d, drz);
             }
             if (F64) rzs = (S) rz;
             pv = fma(by[r], rz, pv);
@@ -366,7 +379,7 @@ __device__ __forceinline__ void bspline_interpolate(const GridView& G, int ix, i
             pdz = fma((S) by[r], drz, pdz);
         }
         val = fma(bx[i], pv, val);
-        gx = fma((S) dbx[i], (S) pv, gx);
+        gx = fma((S) dbx[i], F64 ? (S) pv : (S) (pv - (double) ref), gx);
         gy = fma((S) bx[i], pdy, gy);
         gz = fma((S) bx[i], pdz, gz);
     }
@@ -391,6 +404,7 @@ __device__ __forceinline__ void bspline_interpolate_points(const GridView& G, in
     for (int k = 0; k < 4; k++) zi[k] = min(max(iz - 1 + k, 0), nz - 1);
     val = 0.0;
     gx = gy = gz = (S) 0;
+    S ref = (S) 0;                // MIXED: the stencil's first point, as in bspline_interpolate
 #pragma unroll
     for (int i = 0; i < 4; i++) {
         const size_t px = (size_t) min(max(ix - 1 + i, 0), nx - 1) * ny;
@@ -404,9 +418,11 @@ __device__ __forceinline__ void bspline_interpolate_points(const GridView& G, in
 #pragma unroll
             for (int k = 0; k < 4; k++) {
                 const S v = __ldg(row + zi[k]);
+                if (!F64 && i == 0 && r == 0 && k == 0) ref = v;
+                const S d = F64 ? v : v - ref;
                 rz = fma(bz[k], (double) v, rz);
-                if (!F64) rzs = fma((S) bz[k], v, rzs);
-                drz = fma((S) dbz[k], v, drz);
+                if (!F64) rzs = fma((S) bz[k], d, rzs);
+                drz = fma((S) dbz[k], d, drz);
             }
             if (F64) rzs = (S) rz;
             pv = fma(by[r], rz, pv);
@@ -414,7 +430,7 @@ __device__ __forceinline__ void bspline_interpolate_points(const GridView& G, in
             pdz = fma((S) by[r], drz, pdz);
         }
         val = fma(bx[i], pv, val);
-        gx = fma((S) dbx[i], (S) pv, gx);
+        gx = fma((S) dbx[i], F64 ? (S) pv : (S) (pv - (double) ref), gx);
         gy = fma((S) bx[i], pdy, gy);
         gz = fma((S) bx[i], pdz, gz);
     }
@@ -659,7 +675,8 @@ __global__ void __launch_bounds__(kBlock, eval_min_blocks<S, LAYOUT, NG>()) gf_e
     const unsigned total = (unsigned) p.total;
     const int lane = threadIdx.x & 31;
     const bool active = t < total;
-    if (p.energies_clear && t < (unsigned) (p.n_replicas * p.n_slots)) p.energies_clear[t] = 0.0;
+    if (p.energies_clear)   // grid-stride: with energy slots the next accumulator can have more entries than the launch has threads
+        for (unsigned c = t; c < (unsigned) (p.n_replicas * p.n_slots); c += gridDim.x * blockDim.x) p.energies_clear[c] = 0.0;
 
     int rep = -1;
     unsigned ia = 0;

@@ -189,8 +189,9 @@ def test_f32_force_store_host_path(gpu_device, oracle_built, n_grids, buffers):
 
 @pytest.mark.parametrize("precision", [0, 1], ids=["mixed", "double"])
 def test_f32_force_store_other_kernels_and_subsets(gpu_device, oracle_built, precision):
-    """F32 stores through the general kernel (ROWS layout), the DOUBLE record kernel, the B-spline kernel, and with a
-    particle subset (entries of untouched particles stay as they were)."""
+    """F32 stores with a particle subset (entries of untouched particles stay as they were) through CELLS (the MIXED lines
+    kernel / the DOUBLE record kernel) and ROWS (the general kernel). The B-spline and tricubic record kernels' F32 stores
+    are checked in test_gpu_coverage.py::test_record_kernel_modes."""
     import openmmgridforce_b200 as gf
     rng = np.random.default_rng(8)
     r, n_particles, a = 7, 90, 60
